@@ -8,6 +8,8 @@ MLP Problem (BASELINE.json configs[1] at N=1, configs[2] at N>1; batch 4096 per 
                                                              # torch.optim (+ DDP at N>1), the
                                                              # "kernel to beat" of SURVEY §8(d)
     python bench.py --workload resnet18|resnet50x4 ...       # BASELINE configs[3] / configs[4]
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's
+                                                             # outputs as DIR/*.npy (float32)
 
 One JSON line on stdout (rank 0).  Everything else goes to stderr.
 """
@@ -59,7 +61,12 @@ def parse_args():
     ap.add_argument("--graph", type=int, default=1, help="replay the step from a CUDA graph (1) or issue it eagerly (0)")
     ap.add_argument("--profile", default=None,
                     help="write a JSON summary (device time per kernel per step, torch.profiler over 5 steps) here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="b200 arm: after the timed steps, write what the last timed step returned (model "
+                         "outputs, losses) and a fixed sample of the master weights it left as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs is implemented for --impl b200 only")
     wl = WORKLOADS[args.workload]
     if args.algo is None:
         args.algo = wl["algo"]
@@ -623,6 +630,37 @@ def nvls_parity_check(worker, step_fn, world, algo, precision):
     return res
 
 
+DUMP_MAX_ELEMS = 1 << 22          # 16 MB of float32 per array: about 34 MB in all for the mlp workload
+
+
+def dump_outputs(out_dir, result, master):
+    """Write what one training step returned to its caller (per-task model outputs, total and
+    per-task losses) and the master weights it left, as float32 ``out_dir/<name>.npy``.  An array
+    of more than DUMP_MAX_ELEMS elements is replaced by the elements at a fixed seeded sample of
+    flat indices (``<name>_sample.npy``), so that two builds can be compared file by file."""
+    import re
+    import numpy as np
+    import torch
+    output, total_loss, sub_loss, _ = result
+    arrays = {"loss_total": total_loss}
+    arrays.update(("loss_" + re.sub(r"[^\w.-]", "_", k), v) for k, v in sub_loss.items())
+    arrays.update(("output_%d" % i, o) for i, o in enumerate(output))
+    arrays["master_weights"] = master
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach().reshape(-1)
+        if t.numel() > DUMP_MAX_ELEMS:
+            gen = torch.Generator().manual_seed(0)
+            idx = torch.randperm(t.numel(), generator=gen)[:DUMP_MAX_ELEMS].sort().values
+            t, name = t[idx.to(t.device)], name + "_sample"
+        a = t.float().cpu().numpy()
+        total += a.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    assert total <= 64 << 20, total
+    log("dumped %d arrays (%.1f MB) of the last timed step to %s" % (len(arrays), total / 2 ** 20, out_dir))
+
+
 def main_b200(args, rank, local_rank, world):
     import torch
     import torch.distributed as dist
@@ -684,7 +722,7 @@ def main_b200(args, rank, local_rank, world):
     def step_resident(i):
         data, target = pool[i % POOL]
         worker.criterion.set_step_sink(log_ring.row(i), log_ring.nan_flag)
-        worker._pass_one_minibatch(i, t.Split.TRAIN, data, target)
+        return worker._pass_one_minibatch(i, t.Split.TRAIN, data, target)
 
     # ======================= leg 1: inputs resident in HBM =======================
     # spin-up: a GPU that sat idle (every GPU but the first on a fresh multi-GPU box) needs tens of
@@ -709,10 +747,13 @@ def main_b200(args, rank, local_rank, world):
         marks[0].record()
         host_t0 = time.perf_counter()
         for i in range(K):
-            step_resident(W + i)
+            last = step_resident(W + i)
             marks[i + 1].record()
         host_issue_ms = 1e3 * (time.perf_counter() - host_t0) / K     # CPU time to ISSUE a step
         barrier()
+    if args.dump_outputs and rank == 0:
+        # before any further step: under graph replay the returned tensors are the graph's buffers
+        dump_outputs(args.dump_outputs, last, arena.master)
     launches = _native.launch_count() + graph_step.REPLAYED_LAUNCHES - launches0
     worker.pipeline.record_update_events = False
     total_ms = marks[0].elapsed_time(marks[K])

@@ -3,7 +3,7 @@
 TEST INFRASTRUCTURE.  Source: ``/root/reference`` where it exists (the build container), else the
 archive ``oracle/build_ref.py`` packed into the git-ignored ``oracle/_ref/reference.zip`` (which
 travels to the GPU box); used by ``oracle/make_golden.py`` to generate the committed fixtures, by
-the ``-m reference`` tests that pin ``oracle/ref_loop.py`` against the live reference and by the
+``oracle/reference_cases.py`` to record the reference's API-parity results, and by the
 CPU arm of ``bench.py``.
 
 What the shim does (SURVEY §8c), without touching the reference tree:

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
@@ -57,3 +59,30 @@ def test_resnet_workload_reference_arm(tmp_path):
     assert out.returncode == 0, out.stderr[-2000:]
     d = json.loads([l for l in out.stdout.splitlines() if l.strip()][-1])
     assert "ResNet-18" in d["config"]["workload"] and d["value"] > 0
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    """--dump-outputs: float32 .npy files of what the last timed step returned, under 64 MB, and
+    the same files from a second run with the same arguments."""
+    import numpy as np
+    dumps = []
+    for run in range(2):
+        d = tmp_path / ("run%d" % run)
+        out = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--gpus", "1", "--steps", "3",
+                              "--warmup", "1", "--batch", "256", "--no-e2e", "--no-torch-baseline",
+                              "--no-cpu-baseline", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=900, cwd=REPO)
+        assert out.returncode == 0, out.stderr[-3000:]
+        line = json.loads([l for l in out.stdout.splitlines() if l.strip()][-1])
+        assert line["steps"] == 3 and line["warmup"] == 1
+        dumps.append({p.name: np.load(p) for p in sorted(d.iterdir())})
+    first, second = dumps
+    assert set(first) == {"loss_total.npy", "loss_cls.npy", "loss_reg.npy", "output_0.npy", "output_1.npy",
+                          "master_weights_sample.npy"}, sorted(first)
+    assert sum(a.nbytes for a in first.values()) <= 64 << 20
+    assert first["output_0.npy"].size == 256 * 1000 and first["output_1.npy"].size == 256 * 64
+    assert first["master_weights_sample.npy"].size == 1 << 22
+    for name, a in first.items():
+        assert a.dtype == np.float32 and np.isfinite(a).all(), name
+        np.testing.assert_array_equal(a, second[name], err_msg=name)

@@ -6,7 +6,8 @@
 * the reference's own tests for this path (tests/test_indexed_dataset.py: header synthesised by
   hand with magic 0 / version 1, write->read round trip, reader survives pickling into another
   process) are restated against this repo's classes;
-* with /root/reference present, writer and reader are compared live on random frames;
+* writer bytes and reader frames on random frames are compared with what the reference's
+  writer and reader produced for them (oracle/reference_cases.py);
 * the batched path: ``host_fields`` (zero-copy [N, ...] tensors over the mapped .bin) gathered by
   the native host pool equals per-sample ``__getitem__`` + stacking.
 """
@@ -26,6 +27,7 @@ import torch
 import frl_b200  # noqa: F401
 from frl_b200 import _native
 from frl_b200 import indexed_dataset as idm
+from oracle import reference_cases as rc
 from oracle.make_indexed_golden import FILES, frames_of
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "indexed")
@@ -161,36 +163,23 @@ def test_malformed_index_files_are_rejected(tmp_path):
         r._init_from_index_data(bad)
 
 
-# ---- live comparison with the reference (build container only) -------------------------------------
+# ---- against what the reference's writer and reader did (oracle/reference_cases.py) ----------------
 
-@pytest.mark.reference
 def test_writer_and_reader_match_the_live_reference(tmp_path):
-    from oracle.ref_shim import import_reference
-    import_reference()
-    from frldistml.scaffold.storage import StoragePath
-    from frldistml.scaffold.storage_layers.dataset import IndexedDatasetWriter as RefWriter
-    from frldistml.scaffold.storage_layers.posix_storage import PosixIndexedDatasetReader as RefReader
-    rs = np.random.RandomState(7)
-    for dt, shape, n in [("float32", (3, 4), 5), ("uint8", (2, 3, 5), 7), ("int64", (), 4),
-                         ("float64", (128,), 3), ("int16", (1,), 1), ("int8", (4, 1, 2), 9),
-                         ("int32", (17,), 33)]:
-        frames = [np.asarray(rs.randn(*shape) * 50).astype(dt) for _ in range(n)]
-        mine_i, mine_b, ref_i, ref_b = io.BytesIO(), io.BytesIO(), io.BytesIO(), io.BytesIO()
-        w, rw = idm.IndexedDatasetWriter(idxfile=mine_i, binfile=mine_b), RefWriter(idxfile=ref_i, binfile=ref_b)
-        for f in frames:
-            w.push_back(f)
-            rw.push_back(f)
-        w.flush()
-        rw.flush()
-        assert mine_i.getvalue() == ref_i.getvalue() and mine_b.getvalue() == ref_b.getvalue(), (dt, shape)
+    want = rc.load("indexed_writer_reader")
+    cases = rc.indexed_frames()
+    assert len(want) == len(cases)
+    for (dt, shape, frames), ref in zip(cases, want):
+        mine_i, mine_b = rc.write_indexed(idm.IndexedDatasetWriter, frames)
+        assert mine_i == bytes(ref["idx"].tolist()) and mine_b == bytes(ref["bin"].tolist()), (dt, shape)
         idx, binf = str(tmp_path / "x.idx"), str(tmp_path / "x.bin")
-        open(idx, "wb").write(ref_i.getvalue())
-        open(binf, "wb").write(ref_b.getvalue())
+        open(idx, "wb").write(mine_i)
+        open(binf, "wb").write(mine_b)
         mine = idm.PosixIndexedDatasetReader(idxfile=idx, binfile=binf)
-        ref = RefReader(idxfile=StoragePath(idx), binfile=StoragePath(binf))
-        assert len(mine) == len(ref) and mine.framesize == ref.framesize and mine.dtype == ref.dtype
-        for i in range(n):
-            a, b = mine[i], ref[i]
+        assert len(mine) == ref["len"] == len(frames)
+        assert mine.framesize == ref["framesize"] and mine.dtype == np.dtype(ref["dtype"])
+        for i in range(len(frames)):
+            a, b = mine[i], ref["frames"][i].numpy()
             assert a.dtype == b.dtype and a.shape == b.shape and np.array_equal(a, b)
 
 
@@ -231,48 +220,17 @@ def test_batched_access_refuses_ragged_files(tmp_path):
 
 # ---- Concat / Subset containers over indexed datasets (reference dataset.py:518-552) ---------------
 
-@pytest.mark.reference
 def test_concat_and_subset_containers_match_the_live_reference(tmp_path):
-    from oracle.ref_shim import import_reference
-    import_reference()
-    import frldistml.scaffold.storage_layers.dataset as ref_ds
-    from frldistml.scaffold.indexed_dataset import MultifieldIndexedDataset as RefMulti
-    from frldistml.scaffold.storage import StoragePath
     import frl_b200.storage_layers.dataset as my_ds
-    rs = np.random.RandomState(9)
-    sizes = [5, 1, 7]
-    for k, n in enumerate(sizes):
-        idm.write_fields(str(tmp_path / ("part%d" % k)),
-                         {"a": rs.randn(n, 3).astype(np.float32), "b": rs.randint(0, 9, (n, 2)).astype(np.int64)})
-
-    class Recorder:
-        def __init__(self, log, offset=0, field=None):
-            self.log, self.offset, self.field = log, offset, field
-
-        def with_dataset_global_offset(self, offset):
-            return Recorder(self.log, offset, self.field)
-
-        def with_multifield_dataset_field(self, field):
-            self.log.append((self.offset, field))
-            return Recorder(self.log, self.offset, field)
-
-    mine_parts = [idm.MultifieldIndexedDataset(str(tmp_path / ("part%d" % k)), fields=["a", "b"], filenames=["a", "b"])
-                  for k in range(3)]
-    ref_parts = [RefMulti(StoragePath(str(tmp_path / ("part%d" % k))), fields=["a", "b"], filenames=["a", "b"])
-                 for k in range(3)]
-    mine, ref = my_ds.ConcatMultifieldDataset(mine_parts), ref_ds.ConcatMultifieldDataset(ref_parts)
-    assert len(mine) == len(ref) == sum(sizes)
-    for i in range(len(ref)):
-        a, b = mine.get_raw_item(i), ref.get_raw_item(i)
-        assert list(a) == list(b) and all(np.array_equal(a[k], b[k]) and a[k].dtype == b[k].dtype for k in a)
-        c, d = mine[i], ref[i]
-        assert all(np.array_equal(c[k], d[k]) for k in c)
-    log_mine, log_ref = [], []
-    mine.set_accessor(Recorder(log_mine))
-    ref.set_accessor(Recorder(log_ref))
-    assert log_mine == log_ref == [(0, "a"), (0, "b"), (5, "a"), (5, "b"), (6, "a"), (6, "b")]
-    picks = [12, 0, 5, 5, 3]
-    sub_mine, sub_ref = my_ds.SubsetMultifieldDataset(mine, picks), ref_ds.SubsetMultifieldDataset(ref, picks)
-    assert len(sub_mine) == len(sub_ref) == 5
-    for j in range(5):
-        assert all(np.array_equal(sub_mine[j][k], sub_ref[j][k]) for k in ("a", "b"))
+    ref = rc.load("concat_subset")
+    rc.write_concat_parts(str(tmp_path))
+    parts = [idm.MultifieldIndexedDataset(str(tmp_path / ("part%d" % k)), fields=["a", "b"], filenames=["a", "b"])
+             for k in range(3)]
+    mine = rc.concat_and_subset(my_ds.ConcatMultifieldDataset(parts), my_ds.SubsetMultifieldDataset)
+    assert mine["len"] == ref["len"] == 13
+    for key in ("raw", "items", "subset"):
+        assert len(mine[key]) == len(ref[key])
+        for a, b in zip(mine[key], ref[key]):
+            assert list(a) == list(b) and all(torch.equal(a[k], b[k]) and a[k].dtype == b[k].dtype for k in a), key
+    assert mine["accessor_log"] == ref["accessor_log"] == [(0, "a"), (0, "b"), (5, "a"), (5, "b"), (6, "a"), (6, "b")]
+    assert mine["subset_len"] == ref["subset_len"] == 5

@@ -1,6 +1,6 @@
 """The oracle (oracle/ref_loop.py, optim_np.py, criteria_np.py) against the committed golden
-vectors recorded from the live reference, against the reference itself where it is present,
-and against torch's own ops."""
+vectors recorded from the live reference and against torch's own ops; this package's classes
+against what the reference's classes returned on the same inputs (oracle/reference_cases.py)."""
 import json
 import os
 import re
@@ -10,6 +10,7 @@ import pytest
 import torch
 
 from oracle import criteria_np, optim_np, ref_loop
+from oracle import reference_cases as rc
 from oracle.make_golden import BATCH, CONFIGS, SEED, run_oracle
 
 
@@ -62,11 +63,10 @@ def test_sampler_restatement_matches_reference_lists(golden_dir):
             assert got == expect, key
 
 
-@pytest.mark.reference
-def test_ref_loop_equals_live_reference_bitwise():
-    from oracle.make_golden import run_live_reference
+def test_ref_loop_equals_live_reference_bitwise(golden_dir):
+    """tests/golden/toy_sgd.npz holds what the reference's own LocalSolver.solve recorded."""
     name = "toy_sgd"
-    live = run_live_reference(name, CONFIGS[name])
+    live = _golden_rows(golden_dir, name)
     trace, _ = run_oracle(name, CONFIGS[name])
     rows = np.concatenate([trace.losses[k] for k in sorted(
         trace.losses, key=lambda ek: (ek[0], 0 if ek[1] == "training" else 1))])
@@ -155,156 +155,61 @@ def test_bf16_round_matches_torch():
 
 # ------------------------------------------------------------------------------------------------
 # SURVEY §8 a16 — SamplerState (retained minibatches -> per-sample metrics, random picks, worst-k)
-# against the live reference class on identical inputs
+# against what the reference class returned on identical inputs (oracle/reference_cases.py)
 # ------------------------------------------------------------------------------------------------
 
-@pytest.mark.reference
-@pytest.mark.parametrize("metric_name,ordering", [("err_MSE", "DESC"), ("score", "ASC"), ("score", "DESC")])
+@pytest.mark.parametrize("metric_name,ordering", rc.SAMPLER_STATE_CONFIGS)
 def test_sampler_state_matches_live_reference(metric_name, ordering):
     import random
-    from typing import NamedTuple
-    from oracle.ref_shim import import_reference
-    import_reference()
-    import frldistml.scaffold.solver_worker as ref_sw
-    from frldistml.scaffold.problem import Ordering as RefOrdering
+    from oracle import make_sampler_state_golden as gen
     import frl_b200  # noqa: F401
     import frl_b200.solver_worker as my_sw
     from frl_b200.problem import Ordering as MyOrdering
 
-    class Meta(NamedTuple):
-        index: object = None
+    ref = rc.load("sampler_state_%s_%s" % (metric_name, ordering))
+    batches, total = gen.scenario()
+    random.seed(gen.PY_SEED)
+    state = my_sw.SamplerState(gen.make_problem(MyOrdering, metric_name, ordering), total, total,
+                               torch.device("cpu"), gen.N_VIS)
+    gen.drive(state, batches)
+    state.finish()
+    mine = rc.sampler_state_record(state)
 
-    def make_problem(Ordering):
-        class P:
-            def refine_batch_meta(self, meta):
-                return Meta(**meta)
-
-            def compute_batch_metrics(self, meta, target, output, device):
-                err = ((output[0] - target[0][0]) ** 2).mean(1).numpy()
-                score = (output[1][:, 0] - target[1][0].float()).numpy()      # signed, tie-free
-                return {"err_MSE": err, "score": score}
-
-            def get_rankable_metric(self):
-                return metric_name, Ordering[ordering]
-        return P()
-
-    g = torch.Generator().manual_seed(11)
-    sizes = [16, 16, 16, 16, 9]                       # ragged last minibatch
-    batches, start = [], 0
-    for n in sizes:
-        batches.append(dict(
-            meta={"index": torch.arange(start, start + n)},
-            data=[torch.randn(n, 5, generator=g)],
-            outputs=[torch.randn(n, 4, generator=g), torch.randn(n, 3, generator=g)],
-            targets=[(torch.randn(n, 4, generator=g),), (torch.randint(0, 3, (n,), generator=g),)]))
-        start += n
-    total = start
-
-    class FakeLoader:
-        sampler = list(range(total))
-
-    dev = torch.device("cpu")
-    random.seed(5)
-    ref = ref_sw.SamplerState(make_problem(RefOrdering), FakeLoader, list(range(total)), dev, 6)
-    random.seed(5)
-    mine = my_sw.SamplerState(make_problem(MyOrdering), total, total, dev, 6)
-    for s in (ref, mine):
-        for k, b in enumerate(batches):
-            if k % 2 == 0:                            # amortisation: fold every second minibatch
-                s.compute_metrics()
-            s.append_sample(b["meta"], b["data"], outputs=b["outputs"], targets=b["targets"])
-        s.compute_metrics()
-    mine.finish()
-
-    assert mine.n_samples == ref.n_samples == total
+    assert mine["n_samples"] == ref["n_samples"] == total
     for k in ("err_MSE", "score"):
-        np.testing.assert_array_equal(np.asarray(mine.data_metric[k]), np.asarray(ref.data_metric[k]))
-
-    def ids(samples):
-        return [int(s.meta["index"]) for s in samples]
-
-    assert ids(mine.random_samples) == ids(ref.random_samples) and len(ids(ref.random_samples)) == 6
-    assert sorted(ids(mine.worst_samples)) == sorted(ids(ref.worst_samples))
-    assert len(ref.worst_samples) == 6
-    by_id = {int(s.meta["index"]): s for s in ref.worst_samples + ref.random_samples}
-    for s in mine.worst_samples + mine.random_samples:
-        r = by_id[int(s.meta["index"])]
-        assert all(torch.equal(a, b) for a, b in zip(s.data, r.data))
-        assert all(torch.equal(a, b) for a, b in zip(s.output, r.output))
-        assert all(torch.equal(a[0], b[0]) for a, b in zip(s.target, r.target))
-        assert {k: float(v) for k, v in s.metric.items()} == {k: float(v) for k, v in r.metric.items()}
+        np.testing.assert_array_equal(mine["data_metric"][k].numpy(), ref["data_metric"][k].numpy())
+    assert mine["random_ids"] == ref["random_ids"] and len(ref["random_ids"]) == 6
+    assert sorted(mine["worst_ids"]) == sorted(ref["worst_ids"])
+    assert len(ref["worst_ids"]) == 6
+    for i, s in mine["samples"].items():
+        r = ref["samples"][i]
+        for key in ("data", "output", "target"):
+            assert len(s[key]) == len(r[key]) and all(torch.equal(a, b) for a, b in zip(s[key], r[key])), key
+        assert s["metric"] == r["metric"]
 
 
 # ------------------------------------------------------------------------------------------------
 # SURVEY §8 a8-a11 — the criterion classes' own composition (what runs for arbitrary user losses,
-# and what the fused kernels are checked against on the GPU) against the live reference classes
+# and what the fused kernels are checked against on the GPU) against what the reference classes
+# computed (oracle/reference_cases.py)
 # ------------------------------------------------------------------------------------------------
 
-@pytest.mark.reference
-@pytest.mark.parametrize("kind", ["parallel", "uncertainty", "gradnorm", "masked"])
+@pytest.mark.parametrize("kind", rc.CRITERION_KINDS)
 def test_criterion_classes_match_live_reference(kind):
-    from oracle.ref_shim import import_reference
-    import_reference()
-    import frldistml.scaffold.criteria as ref_c
-    import frldistml.scaffold.model as ref_m
-    import frldistml.scaffold.types as ref_t
     import frl_b200  # noqa: F401
     import frl_b200.criteria as my_c
     import frl_b200.model as my_m
     import frl_b200.types as my_t
 
-    def build(c, m, t):
-        torch.manual_seed(3)
-        trunk = torch.nn.Sequential(m.ListSelect(sel_index=0, num_elements=1), torch.nn.Linear(6, 8),
-                                    torch.nn.ReLU(), torch.nn.Linear(8, 8), torch.nn.ReLU())
-        model = m.MultiTaskModel(trunk, [torch.nn.Linear(8, 3), torch.nn.Linear(8, 5)])
-        mods = [torch.nn.MSELoss(), torch.nn.CrossEntropyLoss()]
-        names, weights = ["reg", "cls"], [0.5, 2.0]
-        if kind == "parallel":
-            crit = c.ParallelCriterion(mods, weights, names)
-        elif kind == "uncertainty":
-            crit = c.UncertaintyWeightedCriterion(
-                mods, [t.LossType.MSE, t.LossType.CrossEntropy], names, weights)
-        elif kind == "gradnorm":
-            crit = c.GradNormWeightedCriterion(mods, names, alpha=1.5, base_weights=weights)
-        else:
-            crit = c.ParallelCriterion([c.MaskedLoss(torch.nn.MSELoss()), torch.nn.CrossEntropyLoss()],
-                                       weights, names)
-        return model, crit
-
-    g = torch.Generator().manual_seed(4)
-    steps = []
-    for k in range(4):
-        x = torch.randn(12, 6, generator=g)
-        y_reg, y_cls = torch.randn(12, 3, generator=g), torch.randint(0, 5, (12,), generator=g)
-        mask = (torch.rand(12, 3, generator=g) > 0.4) if k != 2 else torch.zeros(12, 3, dtype=torch.bool)
-        steps.append((x, y_reg, y_cls, mask))
-
-    def run(c, m, t):
-        model, crit = build(c, m, t)
-        params = list(model.parameters()) + list(crit.parameters())
-        opt = torch.optim.SGD(params, lr=0.05, momentum=0.9)
-        trace = []
-        for x, y_reg, y_cls, mask in steps:
-            out = model([x])
-            if kind == "gradnorm":
-                crit.set_shared_params(model.final_shared_params(out))
-            tgt = [(y_reg, mask) if kind == "masked" else (y_reg,), (y_cls,)]
-            total, sub = crit(out, tgt)
-            opt.zero_grad()
-            total.backward()
-            trace.append((total.detach().clone(), {k: v.detach().clone() for k, v in sub.items()},
-                          [p.grad.detach().clone() for p in params]))
-            opt.step()
-        return trace, [p.detach().clone() for p in params]
-
-    ref_trace, ref_params = run(ref_c, ref_m, ref_t)
-    my_trace, my_params = run(my_c, my_m, my_t)
-    for (rt, rs, rg), (mt, ms, mg) in zip(ref_trace, my_trace):
+    ref = rc.load("criterion_%s" % kind)
+    mine = rc.criterion_trace(kind, my_c, my_m, my_t)
+    assert len(mine["steps"]) == len(ref["steps"]) == 4
+    for (rt, rs, rg), (mt, ms, mg) in zip(ref["steps"], mine["steps"]):
         assert torch.equal(mt, rt)
         assert list(ms) == list(rs) and all(torch.equal(ms[k], rs[k]) for k in rs)
         assert len(mg) == len(rg) and all(torch.equal(a, b) for a, b in zip(mg, rg))
-    assert all(torch.equal(a, b) for a, b in zip(my_params, ref_params))
+    assert len(mine["params"]) == len(ref["params"])
+    assert all(torch.equal(a, b) for a, b in zip(mine["params"], ref["params"]))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -312,49 +217,14 @@ def test_criterion_classes_match_live_reference(kind):
 # weighted means over ranks, MSE -> RMSE renaming, invalid (negative) metrics passed through
 # ------------------------------------------------------------------------------------------------
 
-@pytest.mark.reference
 def test_rank_aggregation_matches_live_reference():
-    from oracle.ref_shim import import_reference
-    import_reference()
-    import frldistml.scaffold.solver as ref_solver
-    import frldistml.scaffold.solver_worker as ref_sw
-    import frldistml.scaffold.types as ref_t
     import frl_b200  # noqa: F401
     import frl_b200.solver as my_solver
     import frl_b200.solver_worker as my_sw
     import frl_b200.types as my_t
 
-    per_rank = [   # (nSamples, losses, metrics) per split, three ranks with unequal sample counts
-        {"training": (100, {"reg": 0.5, "cls": 2.25}, {"reg_MSE": 0.04, "cls_err": 0.25, "pose_MSE_deg": 9.0}),
-         "testing": (10, {"reg": 0.7, "cls": 2.0}, {"reg_MSE": 0.09, "cls_err": 0.5, "pose_MSE_deg": -1.0})},
-        {"training": (60, {"reg": 0.25, "cls": 1.75}, {"reg_MSE": 0.01, "cls_err": 0.125, "pose_MSE_deg": 4.0}),
-         "testing": (30, {"reg": 0.1, "cls": 3.0}, {"reg_MSE": 0.16, "cls_err": 0.75, "pose_MSE_deg": -1.0})},
-        {"training": (7, {"reg": 1.5, "cls": 0.5}, {"reg_MSE": 0.25, "cls_err": 1.0, "pose_MSE_deg": 1.0}),
-         "testing": (3, {"reg": 0.3, "cls": 1.0}, {"reg_MSE": 0.0, "cls_err": 0.0, "pose_MSE_deg": -1.0})},
-    ]
-
-    def run(solver_mod, sw_mod, t):
-        class DS:
-            def __init__(self, split):
-                self.data_type = split
-
-        class P:
-            datasets = [DS(t.Split.TRAIN), DS(t.Split.TEST)]
-
-        fracs = []
-        for rank in per_rank:
-            perf = {t.Split(name): sw_mod.FractionalEpochSplitPerformanceSummary(
-                        nSamples=n, losses=dict(losses), metrics=dict(metrics), samples=[],
-                        worstSamples=[], testIO=[])
-                    for name, (n, losses, metrics) in rank.items()}
-            fracs.append(sw_mod.FractionalPerformanceSummary(
-                epoch=3, modelBuffer=b"", optimizerStateBuffer=b"", performance=perf))
-        ro = t.RunOpts(optim=t.OptimOpts(algo=t.OptAlgorithm.SGD), batchSize=4)
-        out = solver_mod.Solver._aggregate_fractional_results(ro, P(), fracs)
-        return {split.value: (dict(s.losses), dict(s.metrics)) for split, s in out.items()}
-
-    want = run(ref_solver, ref_sw, ref_t)
-    got = run(my_solver, my_sw, my_t)
+    want = rc.load("rank_aggregation")
+    got = rc.aggregate_ranks(my_solver, my_sw, my_t)
     assert got == want
     assert set(want["training"][1]) == {"reg_RMSE", "cls_err", "pose_RMSE_deg"}
     assert want["testing"][1]["pose_RMSE_deg"] == -1.0          # invalid metric: not square-rooted
@@ -365,65 +235,19 @@ def test_rank_aggregation_matches_live_reference():
 # contents, and each side's loader reads the other's checkpoint
 # ------------------------------------------------------------------------------------------------
 
-@pytest.mark.reference
 def test_checkpoint_files_match_live_reference(tmp_path):
-    import io
-    from typing import NamedTuple
-    from oracle.ref_shim import import_reference
-    import_reference()
-    import frldistml.scaffold.solver as ref_solver
-    import frldistml.scaffold.solver_worker as ref_sw
-    import frldistml.scaffold.types as ref_t
-    from frldistml.scaffold.storage import StoragePath
     import frl_b200  # noqa: F401
     import frl_b200.solver as my_solver
     import frl_b200.solver_worker as my_sw
     import frl_b200.types as my_t
 
-    torch.manual_seed(1)
-    model = torch.nn.Sequential(torch.nn.Linear(6, 5), torch.nn.BatchNorm1d(5), torch.nn.ReLU(),
-                                torch.nn.Linear(5, 3))
-    opt = torch.optim.SGD(model.parameters(), lr=0.1, momentum=0.9, weight_decay=1e-5)
-    for _ in range(3):
-        opt.zero_grad()
-        model(torch.randn(8, 6)).square().mean().backward()
-        opt.step()
-    model.eval()
-    buf = io.BytesIO()
-    torch.save(model, buf)
-    model_bytes = buf.getvalue()
-    buf = io.BytesIO()
-    torch.save(opt.state_dict(), buf)
-    optim_bytes = buf.getvalue()
-    samples = [dict(data=[torch.randn(6)], target=[(torch.randn(3),)], meta={"index": torch.tensor(i)},
-                    output=[torch.randn(3)], metric={"m": 0.5}) for i in range(2)]
-
-    class Anno(NamedTuple):
-        scale: float = 2.0
-        names: tuple = ("a", "b")
-
-    class P:
-        anno_param = Anno()
-
-    def write(solver_mod, sw_mod, t, save_dir):
-        io_samples = [sw_mod.SingleSample(**s) for s in samples]
-        perf = {t.Split.TRAIN: sw_mod.FractionalEpochSplitPerformanceSummary(
-                    nSamples=10, losses={}, metrics={}, samples=[], worstSamples=[], testIO=[]),
-                t.Split.TEST: sw_mod.FractionalEpochSplitPerformanceSummary(
-                    nSamples=4, losses={}, metrics={}, samples=[], worstSamples=[], testIO=io_samples)}
-        frac = sw_mod.FractionalPerformanceSummary(epoch=7, modelBuffer=model_bytes,
-                                                   optimizerStateBuffer=optim_bytes, performance=perf)
-        ro = t.RunOpts(optim=t.OptimOpts(algo=t.OptAlgorithm.SGD), batchSize=4)
-        solver_mod.Solver._save_checkpoint(7, save_dir, ro, P(), [frac], ".checkpoint.pth")
-
-    ref_dir, my_dir = tmp_path / "ref", tmp_path / "mine"
-    ref_dir.mkdir()
+    # the reference's files, written from these very inputs
+    ref_dir, my_dir = rc.CHECKPOINT_DIR, tmp_path / "mine"
     my_dir.mkdir()
-    write(ref_solver, ref_sw, ref_t, StoragePath(str(ref_dir)))
-    write(my_solver, my_sw, my_t, str(my_dir))
-    names = sorted(os.listdir(ref_dir))
-    assert sorted(os.listdir(my_dir)) == names == [".checkpoint.pth", ".checkpoint.pth.annotate_param",
-                                                   ".checkpoint.pth.model", ".checkpoint.pth.test_data"]
+    rc.write_checkpoint(my_solver, my_sw, my_t, str(my_dir), rc.stored_checkpoint_inputs())
+    names = sorted(os.listdir(my_dir))
+    assert names == rc.CHECKPOINT_FILES == [".checkpoint.pth", ".checkpoint.pth.annotate_param",
+                                            ".checkpoint.pth.model", ".checkpoint.pth.test_data"]
 
     def same(a, b):
         if torch.is_tensor(a):
@@ -441,100 +265,57 @@ def test_checkpoint_files_match_live_reference(tmp_path):
     whole_ref = torch.load(os.path.join(ref_dir, ".checkpoint.pth.model"), weights_only=False)
     whole_mine = torch.load(os.path.join(my_dir, ".checkpoint.pth.model"), weights_only=False)
     assert same(dict(whole_ref.state_dict()), dict(whole_mine.state_dict()))
-    # each loader reads the other side's file
-    with open(os.path.join(my_dir, ".checkpoint.pth"), "rb") as f:
-        got = ref_solver.Solver._load_checkpoint(f)
+    # this package's loader reads the reference's file; the reference's loader returns the
+    # "epoch", "state_dict" and "optimizer" entries of what torch.load reads, and those entries of
+    # this package's file were found equal to the reference's above
     with open(os.path.join(ref_dir, ".checkpoint.pth"), "rb") as f:
         back = my_solver.Solver._load_checkpoint(f)
-    assert got.epoch == back.epoch == 7
+    with open(os.path.join(my_dir, ".checkpoint.pth"), "rb") as f:
+        got = my_solver.Solver._load_checkpoint(f)
+    ref_ckpt = torch.load(os.path.join(ref_dir, ".checkpoint.pth"), weights_only=False)
+    assert got.epoch == back.epoch == ref_ckpt["epoch"] == 7
     assert same(dict(got.modelState), dict(back.modelState)) and same(got.optimizerState, back.optimizerState)
+    assert same(dict(back.modelState), dict(ref_ckpt["state_dict"])) and same(back.optimizerState, ref_ckpt["optimizer"])
     torch.optim.SGD(whole_mine.parameters(), lr=0.1, momentum=0.9).load_state_dict(got.optimizerState)
 
 
-@pytest.mark.reference
 def test_initial_model_loading_matches_live_reference(tmp_path, capsys):
     """``initialModelPath`` (reference solver.py:122-159): strict load, and the partial load that
     copies what matches in name and shape and reports the rest — same weights, same messages."""
-    from oracle.ref_shim import import_reference
-    import_reference()
-    import frldistml.scaffold.solver as ref_solver
     import frl_b200  # noqa: F401
     import frl_b200.solver as my_solver
 
-    def net(width):
-        torch.manual_seed(width)
-        return torch.nn.Sequential(torch.nn.Linear(4, width), torch.nn.ReLU(), torch.nn.Linear(width, 2))
-
-    donor = net(5)
-    state = dict(donor.state_dict())
-    state["extra.weight"] = torch.ones(3)
-    state["0.weight"] = torch.nn.Parameter(state["0.weight"].clone())      # legacy serialised Parameter
     path = str(tmp_path / "init.pth")
-    torch.save({"state_dict": state}, path)
-    results = []
-    for mod in (ref_solver, my_solver):
-        target = net(5)
-        del_key = net(7)                       # different width: shape mismatches on every tensor but one
-        mod._load_model_state(target, path, strict=False)
-        mod._load_model_state(del_key, path, strict=False)
-        out = capsys.readouterr().out
-        lines = [l for l in out.splitlines() if l.startswith("Warning")]
-        results.append((dict(target.state_dict()), dict(del_key.state_dict()), lines))
-        with pytest.raises(RuntimeError):
-            mod._load_model_state(net(5), path, strict=True)               # unexpected key "extra.weight"
-        capsys.readouterr()
-    (ra, rb, rl), (ma, mb, ml) = results
+    rc.write_initial_model(path)
+    want = rc.load("initial_model_loading")
+    got = rc.initial_model_loads(my_solver._load_model_state, path, lambda: capsys.readouterr().out)
+    ra, rb, rl = want["target"], want["other"], want["warnings"]
+    ma, mb, ml = got["target"], got["other"], got["warnings"]
+    assert list(ma) == list(ra) and list(mb) == list(rb)
     assert all(torch.equal(ra[k], ma[k]) for k in ra) and all(torch.equal(rb[k], mb[k]) for k in rb)
     assert ml == rl and len(rl) >= 4
-    assert torch.equal(ma["0.weight"], donor.state_dict()["0.weight"])
+    assert got["strict_raises"] and want["strict_raises"]              # unexpected key "extra.weight"
+    assert torch.equal(ma["0.weight"], rc.init_net(5).state_dict()["0.weight"])
 
 
-@pytest.mark.reference
 def test_multitask_problem_plumbing_matches_live_reference():
     """The same synthetic MultiTaskProblem source instantiated against this package and against
     the reference (SURVEY §8b: Problem/MultiTaskProblem/MultiTaskTransform/Task/MultiTaskModel):
     per-sample items, model structure and initial weights, criterion composition, merged metric
     hooks and rankable metric must coincide."""
-    from oracle.ref_shim import import_reference
-    import_reference()
-    import frl_b200  # noqa: F401
-    from frl_b200 import synthetic
-    built = {}
-    for pkg in ("frldistml.scaffold", "frl_b200"):
-        ns = synthetic.api_namespace(pkg)
-        problem = synthetic.make_toy_problem(ns, "/tmp/unused")
-        torch.manual_seed(21)
-        model = problem.get_model()
-        crit = problem.get_criterion()
-        items = [problem.datasets[0][i] for i in (0, 5, 511)] + [problem.datasets[1][3]]
-        g = torch.Generator().manual_seed(2)
-        out = [torch.randn(6, 4, generator=g), torch.randn(6, 10, generator=g)]
-        tgt = [(torch.randn(6, 4, generator=g),), (torch.randint(0, 10, (6,), generator=g),)]
-        meta = problem.refine_batch_meta({"index": torch.arange(6)})
-        metrics = problem.compute_batch_metrics(meta=meta, target=tgt, output=out, device=torch.device("cpu"))
-        with torch.no_grad():
-            y = model([torch.ones(2, 64)])
-        built[pkg] = dict(
-            model_type=type(model).__name__, crit_type=type(crit).__name__,
-            state={k: v.clone() for k, v in model.state_dict().items()},
-            names=list(crit.loss_names), weights=[float(w) for w in crit.loss_weights],
-            loss_mods=[type(m).__name__ for m in crit.loss_modules], items=items,
-            metrics={k: np.asarray(v) for k, v in metrics.items()},
-            rank=(problem.get_rankable_metric()[0], problem.get_rankable_metric()[1].name),
-            epoch=problem.summarize_epoch_metrics({k: np.asarray(v) for k, v in metrics.items()}),
-            meta_fields=meta._fields, y=[t.clone() for t in y],
-            splits=[d.data_type.value for d in problem.datasets], lens=[len(d) for d in problem.datasets])
-    ref, mine = built["frldistml.scaffold"], built["frl_b200"]
+    ref = rc.load("multitask_problem")
+    mine = rc.multitask_problem_plumbing("frl_b200")
     for k in ("model_type", "crit_type", "names", "weights", "loss_mods", "rank", "epoch", "meta_fields",
               "splits", "lens"):
         assert mine[k] == ref[k], k
     assert list(mine["state"]) == list(ref["state"])
     assert all(torch.equal(mine["state"][k], ref["state"][k]) for k in ref["state"])
-    assert all(torch.equal(a, b) for a, b in zip(mine["y"], ref["y"]))
+    assert len(mine["y"]) == len(ref["y"]) and all(torch.equal(a, b) for a, b in zip(mine["y"], ref["y"]))
+    assert list(mine["metrics"]) == list(ref["metrics"])
     assert all(np.array_equal(mine["metrics"][k], ref["metrics"][k]) for k in ref["metrics"])
+    assert len(mine["items"]) == len(ref["items"]) == 4
     for a, b in zip(mine["items"], ref["items"]):
         assert len(a) == len(b) == 3
-        assert all(torch.equal(x, y) for x, y in zip(a[0], b[0]))                      # data list
-        assert all(torch.equal(x[0], y[0]) for x, y in zip(a[1], b[1]))                # target tuples
-        assert list(a[2]) == list(b[2]) and all(torch.equal(torch.as_tensor(a[2][k]), torch.as_tensor(b[2][k]))
-                                                 for k in a[2])
+        assert len(a[0]) == len(b[0]) and all(torch.equal(x, y) for x, y in zip(a[0], b[0]))   # data list
+        assert len(a[1]) == len(b[1]) and all(torch.equal(x[0], y[0]) for x, y in zip(a[1], b[1]))  # targets
+        assert list(a[2]) == list(b[2]) and all(torch.equal(a[2][k], b[2][k]) for k in a[2])
