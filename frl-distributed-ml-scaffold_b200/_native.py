@@ -54,11 +54,13 @@ SIGNATURES = {
     "frl_device_arch": (_i, []),
     "frl_sgd_momentum": (_i, [_vp, _vp, _vp, _vp, _i64, _d, _d, _d, _d, _d, _vp, _vp, _i, _i, _vp]),
     "frl_adam": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _d, _d, _d, _d, _d, _i64, _d, _vp, _vp, _i, _vp]),
+    "frl_adamw": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _d, _d, _d, _d, _d, _i64, _d, _vp, _vp, _i, _vp]),
     "frl_rmsprop": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _d, _d, _d, _d, _d, _d, _vp, _vp, _i, _vp]),
     "frl_mt_tile_elems": (_i64, []),
     "frl_flatten_grads": (_i, [_vp, _vp, _vp, _i64, _vp, _i, _d, _vp]),
     "frl_sgd_momentum_mt": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _d, _d, _d, _d, _d, _vp, _vp, _i, _vp]),
     "frl_adam_mt": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _d, _d, _d, _d, _d, _i64, _d, _vp, _vp, _vp]),
+    "frl_adamw_mt": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _d, _d, _d, _d, _d, _i64, _d, _vp, _vp, _vp]),
     "frl_rmsprop_mt": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _d, _d, _d, _d, _d, _d, _vp, _vp, _vp]),
     "frl_reduce_scratch_bytes": (_i64, []),
     "frl_grad_sumsq_clip": (_i, [_vp, _i64, _i, _f, _f, _vp, _vp, _vp]),
@@ -82,6 +84,8 @@ SIGNATURES = {
     "frl_nvls_sgd": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _vp, _i, _vp, _i, _d, _d, _d, _d, _d, _vp, _i, _i, _i, _vp]),
     "frl_nvls_adam": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _vp, _i, _vp, _i, _d, _d, _d, _d, _d,
                            _i64, _d, _vp, _i, _i, _vp]),
+    "frl_nvls_adamw": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _vp, _i, _vp, _i, _d, _d, _d, _d, _d,
+                            _i64, _d, _vp, _i, _i, _vp]),
     "frl_nvls_rmsprop": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _vp, _i, _vp, _i, _d, _d, _d, _d, _d, _d,
                               _vp, _i, _i, _vp]),
     "frl_nvls_barrier": (_i, [_vp, _i, _i, _i, _vp]),
@@ -170,6 +174,14 @@ def adam(p, g, m, v, vmax, p_lp, n, *, lr, beta1, beta2, eps, wd, step, grad_sca
                           dtype_code(g.dtype), _stream()), "frl_adam")
 
 
+def adamw(p, g, m, v, vmax, p_lp, n, *, lr, beta1, beta2, eps, wd, step, grad_scale=1.0,
+          grad_scale_dev=None, dyn=None) -> None:
+    """``adam`` with decoupled weight decay (torch.optim.AdamW): p *= 1 - lr*wd, g not decayed."""
+    _check(lib().frl_adamw(_ptr(p), _ptr(g), _ptr(m), _ptr(v), _ptr(vmax), _ptr(p_lp), n, lr,
+                           beta1, beta2, eps, wd, step, grad_scale, _ptr(grad_scale_dev), _ptr(dyn),
+                           dtype_code(g.dtype), _stream()), "frl_adamw")
+
+
 def rmsprop(p, g, sq, buf, p_lp, n, *, lr, alpha, eps, wd, mu, grad_scale=1.0,
             grad_scale_dev=None, dyn=None) -> None:
     _check(lib().frl_rmsprop(_ptr(p), _ptr(g), _ptr(sq), _ptr(buf), _ptr(p_lp), n, lr, alpha,
@@ -204,6 +216,13 @@ def adam_mt(p, m, v, vmax, p_lp, table, *, lr, beta1, beta2, eps, wd, step, grad
     _check(lib().frl_adam_mt(_ptr(p), _ptr(m), _ptr(v), _ptr(vmax), _ptr(p_lp), table.segs_dev_ptr,
                              table.prefix_dev_ptr, table.tile_seg_dev_ptr, table.n_tiles, lr, beta1, beta2, eps, wd,
                              step, grad_scale, _ptr(grad_scale_dev), _ptr(dyn), _stream()), "frl_adam_mt")
+
+
+def adamw_mt(p, m, v, vmax, p_lp, table, *, lr, beta1, beta2, eps, wd, step, grad_scale=1.0,
+             grad_scale_dev=None, dyn=None) -> None:
+    _check(lib().frl_adamw_mt(_ptr(p), _ptr(m), _ptr(v), _ptr(vmax), _ptr(p_lp), table.segs_dev_ptr,
+                              table.prefix_dev_ptr, table.tile_seg_dev_ptr, table.n_tiles, lr, beta1, beta2, eps,
+                              wd, step, grad_scale, _ptr(grad_scale_dev), _ptr(dyn), _stream()), "frl_adamw_mt")
 
 
 def rmsprop_mt(p, sq, buf, p_lp, table, *, lr, alpha, eps, wd, mu, grad_scale=1.0, grad_scale_dev=None,
@@ -315,6 +334,15 @@ def nvls_adam(p, m, v, vmax, mc_g, mc_out, n, link, *, lr, beta1, beta2, eps, wd
                                link.world, link.pads_dev, link.pad_base, _ptr(link.scratch), link.max_blocks, lr, beta1,
                                beta2, eps, wd, step, grad_scale, _ptr(dyn), g_dtype, link.flags, _stream()),
            "frl_nvls_adam")
+
+
+def nvls_adamw(p, m, v, vmax, mc_g, mc_out, n, link, *, lr, beta1, beta2, eps, wd, step, grad_scale,
+               g_dtype, dyn=None) -> None:
+    _check(lib().frl_nvls_adamw(_ptr(p), _ptr(m), _ptr(v), _ptr(vmax), mc_g, mc_out, n, link.rank,
+                                link.world, link.pads_dev, link.pad_base, _ptr(link.scratch), link.max_blocks, lr,
+                                beta1, beta2, eps, wd, step, grad_scale, _ptr(dyn), g_dtype, link.flags,
+                                _stream()),
+           "frl_nvls_adamw")
 
 
 def nvls_rmsprop(p, sq, buf, mc_g, mc_out, n, link, *, lr, alpha, eps, wd, mu, grad_scale, g_dtype,

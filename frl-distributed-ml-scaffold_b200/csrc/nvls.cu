@@ -290,6 +290,20 @@ extern "C" int frl_nvls_adam(float* p, float* m, float* v, float* vmax, const vo
                                            local_scratch, max_blocks, grad_scale, dyn, g_dtype, flags, stream, "frl_nvls_adam");
 }
 
+extern "C" int frl_nvls_adamw(float* p, float* m, float* v, float* vmax, const void* mc_g, void* mc_out,
+                              int64_t n, int rank, int world, void* const* signal_pads_dev, int pad_base,
+                              void* local_scratch, int max_blocks, double lr, double beta1, double beta2, double eps, double wd,
+                              int64_t step, double grad_scale, const float* dyn, int g_dtype, int flags, void* stream) {
+    FRL_REQUIRE(m && v && step >= 1, FRL_E_ARG, "frl_nvls_adamw: state/step");
+    if (vmax)
+        return launch_nvls<AdamRule<true, true>, 3>(make_adam_rule<true, true>(lr, beta1, beta2, eps, wd, step), p, m, v,
+                                                    vmax, mc_g, mc_out, n, rank, world, signal_pads_dev, pad_base,
+                                                    local_scratch, max_blocks, grad_scale, dyn, g_dtype, flags, stream, "frl_nvls_adamw");
+    return launch_nvls<AdamRule<false, true>, 2>(make_adam_rule<false, true>(lr, beta1, beta2, eps, wd, step), p, m, v,
+                                                 nullptr, mc_g, mc_out, n, rank, world, signal_pads_dev, pad_base,
+                                                 local_scratch, max_blocks, grad_scale, dyn, g_dtype, flags, stream, "frl_nvls_adamw");
+}
+
 extern "C" int frl_nvls_rmsprop(float* p, float* sq, float* buf, const void* mc_g, void* mc_out, int64_t n,
                                 int rank, int world, void* const* signal_pads_dev, int pad_base,
                                 void* local_scratch, int max_blocks, double lr, double alpha, double eps, double wd, double mu,

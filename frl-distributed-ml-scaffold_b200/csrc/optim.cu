@@ -403,6 +403,24 @@ extern "C" int frl_adam(float* p, const void* g, float* m, float* v, float* vmax
                                              grad_scale_dev, dyn, g_dtype, st, "frl_adam");
 }
 
+// AdamW: the same kernel as frl_adam with the decoupled rule (p *= 1 - lr*wd, g not decayed)
+extern "C" int frl_adamw(float* p, const void* g, float* m, float* v, float* vmax, void* p_lp,
+                         int64_t n, double lr, double beta1, double beta2, double eps, double wd,
+                         int64_t step, double grad_scale, const float* grad_scale_dev,
+                         const float* dyn, int g_dtype, void* stream) {
+    FRL_REQUIRE(m && v, FRL_E_ARG, "frl_adamw: null state");
+    FRL_REQUIRE(step >= 1, FRL_E_ARG, "frl_adamw: step must be >= 1");
+    const float gs = static_cast<float>(grad_scale);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (vmax)
+        return launch_update<AdamRule<true, true>, 3>(make_adam_rule<true, true>(lr, beta1, beta2, eps, wd, step),
+                                                      p, g, m, v, vmax, p_lp, n, gs, grad_scale_dev, dyn,
+                                                      g_dtype, st, "frl_adamw");
+    return launch_update<AdamRule<false, true>, 2>(make_adam_rule<false, true>(lr, beta1, beta2, eps, wd, step),
+                                                   p, g, m, v, nullptr, p_lp, n, gs, grad_scale_dev, dyn,
+                                                   g_dtype, st, "frl_adamw");
+}
+
 extern "C" int frl_rmsprop(float* p, const void* g, float* sq, float* buf, void* p_lp, int64_t n,
                            double lr, double alpha, double eps, double wd, double mu,
                            double grad_scale, const float* grad_scale_dev, const float* dyn,
@@ -477,6 +495,23 @@ extern "C" int frl_adam_mt(float* p, float* m, float* v, float* vmax, void* p_lp
     return launch_update_mt<AdamRule<false>, 2>(make_adam_rule<false>(lr, beta1, beta2, eps, wd, step), p, m, v, nullptr,
                                                 p_lp, segs_dev, tile_prefix_dev, tile_seg_dev, n_tiles, gs,
                                                 grad_scale_dev, dyn, st, "frl_adam_mt");
+}
+
+extern "C" int frl_adamw_mt(float* p, float* m, float* v, float* vmax, void* p_lp, const frl_grad_seg* segs_dev,
+                            const int64_t* tile_prefix_dev, const int32_t* tile_seg_dev, int64_t n_tiles, double lr, double beta1,
+                            double beta2, double eps, double wd, int64_t step, double grad_scale,
+                            const float* grad_scale_dev, const float* dyn, void* stream) {
+    FRL_REQUIRE(m && v, FRL_E_ARG, "frl_adamw_mt: null state");
+    FRL_REQUIRE(step >= 1, FRL_E_ARG, "frl_adamw_mt: step must be >= 1");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const float gs = static_cast<float>(grad_scale);
+    if (vmax)
+        return launch_update_mt<AdamRule<true, true>, 3>(make_adam_rule<true, true>(lr, beta1, beta2, eps, wd, step),
+                                                         p, m, v, vmax, p_lp, segs_dev, tile_prefix_dev, tile_seg_dev,
+                                                         n_tiles, gs, grad_scale_dev, dyn, st, "frl_adamw_mt");
+    return launch_update_mt<AdamRule<false, true>, 2>(make_adam_rule<false, true>(lr, beta1, beta2, eps, wd, step),
+                                                      p, m, v, nullptr, p_lp, segs_dev, tile_prefix_dev, tile_seg_dev,
+                                                      n_tiles, gs, grad_scale_dev, dyn, st, "frl_adamw_mt");
 }
 
 extern "C" int frl_rmsprop_mt(float* p, float* sq, float* buf, void* p_lp, const frl_grad_seg* segs_dev,

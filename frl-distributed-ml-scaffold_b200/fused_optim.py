@@ -3,8 +3,10 @@
 ``create_fused_optimizer`` is the B200 counterpart of the reference's ``_create_optimizer``
 (reference solver.py:162-188): same three algorithms, same hyper-parameter mapping
 (``OptimOpts.momentum`` feeds SGD *and* RMSprop, ``epsilon``/``amsgrad`` feed Adam, weight decay
-is L2-coupled and applies to every parameter).  ``state_dict()`` / ``load_state_dict()`` speak
-torch's per-parameter format so the reference's ``.checkpoint.pth`` files stay interchangeable.
+is L2-coupled and applies to every parameter).  One extension: ``decoupled_weight_decay=True``
+turns Adam into AdamW (``torch.optim.AdamW``), still decaying every parameter.
+``state_dict()`` / ``load_state_dict()`` speak torch's per-parameter format so the reference's
+``.checkpoint.pth`` files stay interchangeable (and an AdamW run's load into ``torch.optim.AdamW``).
 
 Known limitation: the step count (Adam's bias corrections) is ONE number for the whole arena.
 ``torch.optim`` keeps one per parameter and does not advance it for a parameter whose gradient
@@ -270,11 +272,18 @@ class FusedAdam(FusedArenaOptimizer):
     STATE_NAMES = (("exp_avg", "exp_avg"), ("exp_avg_sq", "exp_avg_sq"),
                    ("max_exp_avg_sq", "max_exp_avg_sq"))
 
-    def __init__(self, arena, lr, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, amsgrad=False):
+    def __init__(self, arena, lr, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, amsgrad=False, *,
+                 decoupled_weight_decay=False):
         super().__init__(arena, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay,
                                      amsgrad=amsgrad, maximize=False, foreach=None,
                                      capturable=False, differentiable=False, fused=None,
-                                     decoupled_weight_decay=False))
+                                     decoupled_weight_decay=bool(decoupled_weight_decay)))
+
+    @property
+    def decoupled(self) -> bool:
+        """torch's ``decoupled_weight_decay``: read from the param group at every launch, so a
+        loaded state dict's flag decides, as it does for ``torch.optim.Adam``."""
+        return bool(self.hyper.get("decoupled_weight_decay", False))
 
     def _per_param_extra(self):
         return {"step": torch.tensor(float(self._steps))}
@@ -282,38 +291,59 @@ class FusedAdam(FusedArenaOptimizer):
     def _dyn_values(self):
         h = self.hyper
         step = self._steps + 1
+        lr = float(h["lr"])
         bc1 = 1.0 - float(h["betas"][0]) ** step
         bc2 = 1.0 - float(h["betas"][1]) ** step
-        return (-(float(h["lr"]) / bc1), bc2 ** 0.5)
+        if self.decoupled:
+            return (-(lr / bc1), bc2 ** 0.5, 1.0 - lr * float(h["weight_decay"]))
+        return (-(lr / bc1), bc2 ** 0.5)
 
     def _launch(self, lo, hi, grad_scale, coef):
         h = self.hyper
         p, g, lp = self._slices(lo, hi)
         vmax = self._state("max_exp_avg_sq")[lo:hi] if h["amsgrad"] else None
-        KERNELS.adam(p, g, self._state("exp_avg")[lo:hi], self._state("exp_avg_sq")[lo:hi], vmax,
-                     lp, hi - lo, lr=float(h["lr"]), beta1=float(h["betas"][0]),
-                     beta2=float(h["betas"][1]), eps=float(h["eps"]),
-                     wd=float(h["weight_decay"]), step=self._steps + 1,
-                     grad_scale=grad_scale, grad_scale_dev=coef, dyn=self._dyn)
+        kernel = KERNELS.adamw if self.decoupled else KERNELS.adam
+        kernel(p, g, self._state("exp_avg")[lo:hi], self._state("exp_avg_sq")[lo:hi], vmax,
+               lp, hi - lo, lr=float(h["lr"]), beta1=float(h["betas"][0]),
+               beta2=float(h["betas"][1]), eps=float(h["eps"]),
+               wd=float(h["weight_decay"]), step=self._steps + 1,
+               grad_scale=grad_scale, grad_scale_dev=coef, dyn=self._dyn)
 
     def _launch_mt(self, table, grad_scale):
         h = self.hyper
-        KERNELS.adam_mt(self.arena.master, self._state("exp_avg"), self._state("exp_avg_sq"),
-                        self._state("max_exp_avg_sq") if h["amsgrad"] else None, self.arena.lp, table,
-                        lr=float(h["lr"]), beta1=float(h["betas"][0]), beta2=float(h["betas"][1]),
-                        eps=float(h["eps"]), wd=float(h["weight_decay"]), step=self._steps + 1,
-                        grad_scale=grad_scale, dyn=self._dyn)
+        kernel = KERNELS.adamw_mt if self.decoupled else KERNELS.adam_mt
+        kernel(self.arena.master, self._state("exp_avg"), self._state("exp_avg_sq"),
+               self._state("max_exp_avg_sq") if h["amsgrad"] else None, self.arena.lp, table,
+               lr=float(h["lr"]), beta1=float(h["betas"][0]), beta2=float(h["betas"][1]),
+               eps=float(h["eps"]), wd=float(h["weight_decay"]), step=self._steps + 1,
+               grad_scale=grad_scale, dyn=self._dyn)
 
     def _launch_nvls(self, lo, hi, grad_scale):
         h = self.hyper
         mc_g, mc_out = self._nvls_ptrs(lo)
         vmax = self._state("max_exp_avg_sq")[lo:hi] if h["amsgrad"] else None
-        KERNELS.nvls_adam(self.arena.master[lo:hi], self._state("exp_avg")[lo:hi],
-                          self._state("exp_avg_sq")[lo:hi], vmax, mc_g, mc_out, hi - lo, self.nvls,
-                          lr=float(h["lr"]), beta1=float(h["betas"][0]), beta2=float(h["betas"][1]),
-                          eps=float(h["eps"]), wd=float(h["weight_decay"]), step=self._steps + 1,
-                          grad_scale=grad_scale, g_dtype=KERNELS.dtype_code(self.arena.grad.dtype),
-                          dyn=self._dyn)
+        kernel = KERNELS.nvls_adamw if self.decoupled else KERNELS.nvls_adam
+        kernel(self.arena.master[lo:hi], self._state("exp_avg")[lo:hi],
+               self._state("exp_avg_sq")[lo:hi], vmax, mc_g, mc_out, hi - lo, self.nvls,
+               lr=float(h["lr"]), beta1=float(h["betas"][0]), beta2=float(h["betas"][1]),
+               eps=float(h["eps"]), wd=float(h["weight_decay"]), step=self._steps + 1,
+               grad_scale=grad_scale, g_dtype=KERNELS.dtype_code(self.arena.grad.dtype),
+               dyn=self._dyn)
+
+
+class FusedAdamW(FusedAdam):
+    """``torch.optim.AdamW``: Adam with decoupled weight decay (p *= 1 - lr*wd, the gradient is
+    not decayed).  As in torch, a thin subclass whose flag stays True whatever a loaded state
+    dict says.  The default ``weight_decay`` here is the caller's (``OptimOpts.weightDecay``
+    through ``create_fused_optimizer``); torch's own default of 1e-2 is not substituted."""
+
+    def __init__(self, arena, lr, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, amsgrad=False):
+        super().__init__(arena, lr, betas=betas, eps=eps, weight_decay=weight_decay, amsgrad=amsgrad,
+                         decoupled_weight_decay=True)
+
+    def load_state_dict(self, state_dict: Dict[str, Any]) -> None:
+        super().load_state_dict(state_dict)
+        self.hyper["decoupled_weight_decay"] = True
 
 
 class FusedRMSprop(FusedArenaOptimizer):
@@ -357,8 +387,20 @@ class FusedRMSprop(FusedArenaOptimizer):
                              g_dtype=KERNELS.dtype_code(self.arena.grad.dtype), dyn=self._dyn)
 
 
-def create_fused_optimizer(arena: ParamArena, optim_opts: OptimOpts) -> FusedArenaOptimizer:
-    """Same dispatch and argument mapping as the reference's ``_create_optimizer``."""
+def check_decoupled_weight_decay(optim_opts: OptimOpts, decoupled_weight_decay: bool) -> None:
+    """Decoupled weight decay exists for Adam only (torch 2.11 has no such flag for SGD/RMSprop)."""
+    if decoupled_weight_decay and optim_opts.algo != OptAlgorithm.ADAM:
+        raise ValueError("decoupled_weight_decay=True needs OptimOpts.algo == OptAlgorithm.ADAM "
+                         "(AdamW); got %s" % getattr(optim_opts.algo, "value", optim_opts.algo))
+
+
+def create_fused_optimizer(arena: ParamArena, optim_opts: OptimOpts, *,
+                           decoupled_weight_decay: bool = False) -> FusedArenaOptimizer:
+    """Same dispatch and argument mapping as the reference's ``_create_optimizer``.
+    ``decoupled_weight_decay=True`` with ``OptAlgorithm.ADAM`` gives AdamW, with
+    ``OptimOpts.weightDecay`` as the decoupled coefficient; with any other algorithm it is a
+    ``ValueError``."""
+    check_decoupled_weight_decay(optim_opts, decoupled_weight_decay)
     algo = optim_opts.algo
     if algo == OptAlgorithm.RMSPROP:
         return FusedRMSprop(arena, lr=optim_opts.lr, momentum=optim_opts.momentum,
@@ -367,6 +409,7 @@ def create_fused_optimizer(arena: ParamArena, optim_opts: OptimOpts) -> FusedAre
         return FusedSGD(arena, lr=optim_opts.lr, momentum=optim_opts.momentum,
                         weight_decay=optim_opts.weightDecay)
     if algo == OptAlgorithm.ADAM:
-        return FusedAdam(arena, lr=optim_opts.lr, weight_decay=optim_opts.weightDecay,
-                         eps=optim_opts.epsilon, amsgrad=optim_opts.amsgrad)
+        cls = FusedAdamW if decoupled_weight_decay else FusedAdam
+        return cls(arena, lr=optim_opts.lr, weight_decay=optim_opts.weightDecay,
+                   eps=optim_opts.epsilon, amsgrad=optim_opts.amsgrad)
     raise ValueError("Unknown optimization algorithm type")

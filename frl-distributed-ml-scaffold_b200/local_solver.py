@@ -19,8 +19,8 @@ SYNC_FILE = "/tmp/frl_dist_ml_sync" + "." + pwd.getpwuid(os.getuid()).pw_name
 class LocalSolver:
     @classmethod
     def solve(cls, run_opts: RunOpts, problem: Problem, save_notebook: bool = False,
-              precision: Optional[Precision] = None, graph: Optional[bool] = None
-              ) -> PerformanceSummary:
+              precision: Optional[Precision] = None, graph: Optional[bool] = None,
+              decoupled_weight_decay: bool = False) -> PerformanceSummary:
         if save_notebook:
             logger.warning("save_notebook is not supported by frl_b200 (visualisation only)")
         # a stale rendezvous file from a crashed run would poison the file:// store
@@ -32,6 +32,6 @@ class LocalSolver:
         last: Optional[PerformanceSummary] = None
         for last in Solver.solve(run_opts, problem, group_name=group_name,
                                  init_method="file://" + SYNC_FILE, precision=precision,
-                                 graph=graph):
+                                 graph=graph, decoupled_weight_decay=decoupled_weight_decay):
             pass
         return last

@@ -28,7 +28,7 @@ import torch.nn as nn
 
 from .arena import ParamArena
 from .criteria import BaseParallelCriterion
-from .fused_optim import create_fused_optimizer
+from .fused_optim import check_decoupled_weight_decay, create_fused_optimizer
 from .grad_sync import BufferBroadcaster, GradBucketPipeline
 from .lr_scheduler import DropEpochsScheduler, WarmupMultiStepLR
 from .problem import Problem
@@ -78,6 +78,14 @@ class Checkpoint(NamedTuple):
     optimizerState: Dict[Any, Any]
 
 
+def _update_rule_name(optimizer) -> str:
+    """Name of the update rule in torch's terms, for the one-line path log."""
+    name = type(optimizer).__name__.replace("Fused", "")
+    if name == "Adam" and optimizer.param_groups[0].get("decoupled_weight_decay", False):
+        name = "AdamW"
+    return name + (" (amsgrad)" if optimizer.param_groups[0].get("amsgrad", False) else "")
+
+
 class SolverWorkerArgs(NamedTuple):
     run_opts: RunOpts
     problem: Problem
@@ -94,6 +102,7 @@ class SolverWorkerArgs(NamedTuple):
     precision: Precision = Precision.FP32
     save_every: int = 1
     graph_step: Optional[bool] = None      # None: FRL_B200_CUDA_GRAPH (default off)
+    decoupled_weight_decay: bool = False   # True with OptAlgorithm.ADAM: AdamW
 
 
 def _torch_load(f, **kw):
@@ -309,7 +318,8 @@ class Solver:
             for buf in model.buffers():
                 if buf.is_floating_point():
                     buf.data = buf.data.to(torch.bfloat16)
-        optimizer = create_fused_optimizer(arena, run_opts.optim)
+        optimizer = create_fused_optimizer(arena, run_opts.optim,
+                                           decoupled_weight_decay=args.decoupled_weight_decay)
         if checkpoint:
             optimizer.load_state_dict(checkpoint.optimizerState)
         nvls_link = None
@@ -359,10 +369,10 @@ class Solver:
         if args.rank == 0:
             # one line per run: which of the alternative paths this configuration took
             logger.info(
-                "frl_b200 step: precision %s | step issue %s | gradient exchange %s | update %s | "
-                "Linear layers with arena-born gradients %d (%d fused with their ReLU) | other "
-                "gradients %s",
-                args.precision.value,
+                "frl_b200 step: precision %s | update rule %s | step issue %s | gradient exchange %s | "
+                "update %s | Linear layers with arena-born gradients %d (%d fused with their ReLU) | "
+                "other gradients %s",
+                args.precision.value, _update_rule_name(optimizer),
                 "CUDA-graph replay after 2 eager steps" if worker.graphed is not None else "eager launches",
                 ("fused NVLS kernel per bucket (K7), %d buckets" % len(pipeline.buckets)) if pipeline.nvls is not None
                 else ("ncclAllReduce in place + K2 per bucket, %d buckets" % len(pipeline.buckets)) if distributed
@@ -572,9 +582,9 @@ class Solver:
     @classmethod
     def solve(cls, run_opts: RunOpts, problem: Problem, *, group_name: Optional[str],
               init_method: str, node_idx: int = 0, node_count: int = 1, memory_quota: int = 0,
-              precision: Optional[Precision] = None, graph: Optional[bool] = None
-              ) -> Iterator[PerformanceSummary]:
-        """The reference's entry point (solver.py:728-739) plus two keyword-only extensions:
+              precision: Optional[Precision] = None, graph: Optional[bool] = None,
+              decoupled_weight_decay: bool = False) -> Iterator[PerformanceSummary]:
+        """The reference's entry point (solver.py:728-739) plus three keyword-only extensions:
 
         ``precision``  ``Precision.FP32`` (default; parity with the reference's arithmetic) or
                        ``Precision.BF16`` (bf16 forward/backward/gradients, fp32 master weights and
@@ -583,7 +593,13 @@ class Solver:
                        has run 2 eager steps (the Problem's forward must be capturable: static
                        shapes, no host syncs; a failed capture falls back to eager launches).
                        None: FRL_B200_CUDA_GRAPH (default off).
+        ``decoupled_weight_decay``  True with ``OptimOpts(algo=OptAlgorithm.ADAM)``: AdamW
+                       (``torch.optim.AdamW``; ``OptimOpts.weightDecay`` is the decoupled
+                       coefficient, ``epsilon``/``amsgrad`` as for Adam).  With SGD or RMSprop it
+                       raises ``ValueError`` before any rank starts.  False (default): Adam's
+                       L2-coupled decay, as in the reference.
         """
+        check_decoupled_weight_decay(run_opts.optim, decoupled_weight_decay)
         n_visible = 0 if run_opts.cpuonly else _cuda_device_count_without_poisoning_fork()
         if n_visible == 0:
             raise RuntimeError(
@@ -621,7 +637,8 @@ class Solver:
                 node_idx=node_idx, node_count=node_count,
                 rank=node_idx * device_count + local_rank, local_rank=local_rank,
                 world_size=world_size, group_name=group_name, init_method=init_method,
-                cache=None, precision=prec, save_every=save_every, graph_step=graph)
+                cache=None, precision=prec, save_every=save_every, graph_step=graph,
+                decoupled_weight_decay=decoupled_weight_decay)
             if not run_opts.singleThreaded:
                 parent_conn, child_conn = ctx.Pipe(duplex=False)
                 proc = ctx.Process(target=cls._solver_worker_process,

@@ -83,7 +83,10 @@ class OptimOpts(NamedTuple):
                   arguments (or the device-resident ``dyn`` block under CUDA-graph replay)
     lr_scheduler  ``drop`` or ``multistep`` closed forms, stepped once per epoch
     weightDecay   L2-COUPLED decay folded into the gradient read, on every parameter (model and
-                  criterion) — this is ``torch.optim``'s ``weight_decay``, not AdamW's
+                  criterion) — this is ``torch.optim``'s ``weight_decay``.  With
+                  ``Solver.solve(..., decoupled_weight_decay=True)`` and ADAM it is AdamW's
+                  decoupled coefficient instead (p *= 1 - lr*weightDecay before the Adam step;
+                  the default 1e-5 stays, torch.optim.AdamW's 1e-2 is not substituted)
     momentum      SGD momentum AND RMSprop momentum (the reference feeds both from this field)
     epsilon       Adam only (RMSprop keeps torch's 1e-8), as in the reference's factory
     amsgrad       Adam: adds the running maximum of the second moment (a third state vector)

@@ -42,7 +42,7 @@ int          frl_device_arch(void);
 
 /* ------------------------------------------------------------------------------------------
  * K2 — fused optimizer update over a flat bucket of the parameter arena.
- * Replaces torch.optim.{SGD,Adam,RMSprop}.step() (reference solver.py:162-188, called at
+ * Replaces torch.optim.{SGD,Adam,AdamW,RMSprop}.step() (reference solver.py:162-188, called at
  * solver_worker.py:592) AND the DDP reducer's scale / copy-out passes (reference
  * solver.py:287-289): the reduced gradient is read once, straight from the bucket.
  *
@@ -58,8 +58,11 @@ int          frl_device_arch(void);
  * when it hands Python scalars to fp32 tensor ops.
  *   dyn      optional DEVICE array of per-step scalars that override the by-value arguments,
  *            so a CUDA graph that captured the launch stays valid while they change:
- *            SGD / RMSprop: dyn[0] = lr ;  Adam: dyn[0] = -lr/(1-beta1^t), dyn[1] = sqrt(1-beta2^t).
- * Update rules are torch 2.11's (L2-coupled weight decay: g += wd * p first).
+ *            SGD / RMSprop: dyn[0] = lr ;  Adam: dyn[0] = -lr/(1-beta1^t), dyn[1] = sqrt(1-beta2^t) ;
+ *            AdamW: dyn[0] = -lr/(1-beta1^t), dyn[1] = sqrt(1-beta2^t), dyn[2] = 1-lr*wd.
+ *            The block is 4 floats; a rule reads only its own slots.
+ * Update rules are torch 2.11's: L2-coupled weight decay (g += wd * p first) for SGD, Adam and
+ * RMSprop; decoupled weight decay (p *= 1-lr*wd first, g not decayed) for AdamW.
  * ---------------------------------------------------------------------------------------- */
 
 /* SGD: buf = first_step ? g : mu*buf + (1-dampening)*g ; p -= lr*buf.   mu == 0: buf may be NULL. */
@@ -74,6 +77,14 @@ int frl_adam(float* p, const void* g, float* m, float* v, float* vmax, void* p_l
              double lr, double beta1, double beta2, double eps, double wd, int64_t step,
              double grad_scale, const float* grad_scale_dev, const float* dyn, int g_dtype,
              void* stream);
+
+/* AdamW = torch.optim.AdamW = Adam(decoupled_weight_decay=True): p *= 1-lr*wd (formed in double,
+ * rounded to fp32 once), then the Adam update of the decayed p with the undecayed gradient.
+ * Same arguments, state and traffic as frl_adam; `wd` is the decoupled coefficient. */
+int frl_adamw(float* p, const void* g, float* m, float* v, float* vmax, void* p_lp, int64_t n,
+              double lr, double beta1, double beta2, double eps, double wd, int64_t step,
+              double grad_scale, const float* grad_scale_dev, const float* dyn, int g_dtype,
+              void* stream);
 
 /* RMSprop (not centered): sq = alpha*sq + (1-alpha)*g^2 ; avg = sqrt(sq)+eps ;
  * mu > 0: buf = mu*buf + g/avg ; p -= lr*buf     else: p -= lr*g/avg  (buf may be NULL). */
@@ -119,6 +130,11 @@ int frl_adam_mt(float* p, float* m, float* v, float* vmax, void* p_lp, const frl
                 const int64_t* tile_prefix_dev, const int32_t* tile_seg_dev, int64_t n_tiles, double lr, double beta1,
                 double beta2, double eps, double wd, int64_t step, double grad_scale,
                 const float* grad_scale_dev, const float* dyn, void* stream);
+
+int frl_adamw_mt(float* p, float* m, float* v, float* vmax, void* p_lp, const frl_grad_seg* segs_dev,
+                 const int64_t* tile_prefix_dev, const int32_t* tile_seg_dev, int64_t n_tiles, double lr, double beta1,
+                 double beta2, double eps, double wd, int64_t step, double grad_scale,
+                 const float* grad_scale_dev, const float* dyn, void* stream);
 
 int frl_rmsprop_mt(float* p, float* sq, float* buf, void* p_lp, const frl_grad_seg* segs_dev,
                    const int64_t* tile_prefix_dev, const int32_t* tile_seg_dev, int64_t n_tiles, double lr, double alpha,
@@ -253,6 +269,11 @@ int frl_nvls_adam(float* p, float* m, float* v, float* vmax, const void* mc_g, v
                   void* local_scratch, int max_blocks, double lr, double beta1, double beta2,
                   double eps, double wd,
                   int64_t step, double grad_scale, const float* dyn, int g_dtype, int flags, void* stream);
+int frl_nvls_adamw(float* p, float* m, float* v, float* vmax, const void* mc_g, void* mc_out,
+                   int64_t n, int rank, int world, void* const* signal_pads_dev, int pad_base,
+                   void* local_scratch, int max_blocks, double lr, double beta1, double beta2,
+                   double eps, double wd,
+                   int64_t step, double grad_scale, const float* dyn, int g_dtype, int flags, void* stream);
 int frl_nvls_rmsprop(float* p, float* sq, float* buf, const void* mc_g, void* mc_out, int64_t n,
                      int rank, int world, void* const* signal_pads_dev, int pad_base,
                      void* local_scratch, int max_blocks, double lr, double alpha, double eps,

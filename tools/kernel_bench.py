@@ -59,7 +59,8 @@ def sets_for(bytes_per_set):
 
 def bench_k2(iters):
     out = []
-    for label, n, algo in (("mlp", 54_703_144, "sgd"), ("mlp", 54_703_144, "adam"),
+    # AdamW next to Adam: same bytes (28 B/param), one more multiply per element
+    for label, n, algo in (("mlp", 54_703_144, "sgd"), ("mlp", 54_703_144, "adam"), ("mlp", 54_703_144, "adamw"),
                            ("r18", 11_689_512, "sgd"), ("r50x4", 25_790_618, "adam")):
         n = (n + 7) // 8 * 8
         p = torch.randn(n, device=DEV)
@@ -72,9 +73,8 @@ def bench_k2(iters):
                                      first_step=False)
             bpp = 20
         else:
-            def fn(i, p=p, g=g, s0=s0, s1=s1, lp=lp, n=n):
-                _native.adam(p, g, s0, s1, None, lp, n, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8,
-                             wd=1e-5, step=3)
+            def fn(i, p=p, g=g, s0=s0, s1=s1, lp=lp, n=n, k=getattr(_native, algo)):
+                k(p, g, s0, s1, None, lp, n, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, wd=1e-5, step=3)
             bpp = 28
         out.append(timed("K2 %s %s bf16-grad (%d elems)" % (algo, label, n), fn, 1, bpp * n, iters,
                          "one set: the arena itself is %d MB" % (bpp * n >> 20)))
@@ -92,8 +92,10 @@ def bench_k2mt(iters):
             self.index, self.offset, self.numel = index, offset, numel
 
     out = []
+    r50x4_heads = [(2048, 1000), (2048, 100), (2048, 10), (2048, 4)]
     for label, arch, heads, algo in (("r18", "resnet18", [(512, 1000)], "sgd"),
-                                     ("r50x4", "resnet50", [(2048, 1000), (2048, 100), (2048, 10), (2048, 4)], "adam")):
+                                     ("r50x4", "resnet50", r50x4_heads, "adam"),
+                                     ("r50x4", "resnet50", r50x4_heads, "adamw")):
         net = getattr(torchvision.models, arch)(weights=None)
         sizes = [p.numel() for n, p in net.named_parameters() if not n.startswith("fc.")]
         for i, o in heads:
@@ -118,11 +120,13 @@ def bench_k2mt(iters):
                 _native.sgd_momentum_mt(p, s0, lp, table, lr=0.01, mu=0.9, dampening=0.0, wd=1e-5, first_step=False)
             bpp = 20
         else:
-            def fn(i, p=p, s0=s0, s1=s1, lp=lp, table=table):
-                _native.adam_mt(p, s0, s1, None, lp, table, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, wd=1e-5, step=3)
+            def fn(i, p=p, s0=s0, s1=s1, lp=lp, table=table, k=getattr(_native, algo + "_mt")):
+                k(p, s0, s1, None, lp, table, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, wd=1e-5, step=3)
             bpp = 28
         out.append(timed("K2-mt %s %s: %d tensors, %d params, gradients read in place" % (algo, label, len(sizes), n_real),
                          fn, 1, bpp * n_real, iters))
+        if algo == "adamw":
+            continue                  # same table and gradients as the Adam row: K1 is timed there
         out.append(timed("K1 flatten_grads %s: %d tensors -> bf16 arena, one launch" % (label, len(sizes)),
                          lambda i, table=table, flat=flat: _native.flatten_grads(table, flat, scale=1.0), 1,
                          4 * n_real, iters))
